@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- DSMIL aggregator forward throughput on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 metric  : patches/sec of the DSMIL forward (MILNet.forward, dsmil.py:70-74) at N=10 000, D=512, C=2.
 step    : one pass over a stream of `--bags` synthetic bags (default 16 x 10 000 x 512 fp32 = 328 MB,
@@ -516,6 +516,16 @@ def embed_leg(dev, refmod, batch=128):
     return out
 
 
+def dump_outputs(out_dir, bag_outputs):
+    """Writes what one forward_bags step hands its caller -- per bag (classes, prediction_bag, A, B) -- as float32
+    arrays concatenated over the bags: classes.npy [sum N, C], prediction_bag.npy [bags, C], A.npy [sum N, C],
+    B.npy [bags, C, D].  16 bags of N=10 000 come to 2.6 MB."""
+    os.makedirs(out_dir, exist_ok=True)
+    for i, name in enumerate(("classes", "prediction_bag", "A", "B")):
+        t = torch.cat([o[i] for o in bag_outputs])
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 def run_ours(args):
     import torch.distributed as dist
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -605,10 +615,13 @@ def run_ours(args):
     barrier()
     e0.record()
     for _ in range(args.steps):
-        step()
+        last = step()
     e1.record()
     barrier()
     launches = int(lib.dsmil_launch_count() - l0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
+        del last
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
@@ -892,7 +905,13 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the extra workloads (eager-GPU baseline, N=8192, "
                     "N=15000 training step, N=100k strong scaling, multi-rank parity check)")
     ap.add_argument("--giant-bags", type=int, default=32, help="N=100 000 bags per step of the strong-scaling workload")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step to DIR/<name>.npy "
+                    "(inputs are seeded: two builds run with the same arguments can be compared output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and (args.impl != "ours" or args.gpus != 1 or int(os.environ.get("WORLD_SIZE", "1")) != 1):
+        ap.error("--dump-outputs needs --impl ours on one GPU")
     if args.impl == "reference":
         run_reference(args)
     else:

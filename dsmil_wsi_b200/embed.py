@@ -147,16 +147,21 @@ class _Staging:
         self.stream = torch.cuda.Stream(device=device)
         self.decoder = jpeg.JpegBatchDecoder(device)
 
+    # The device buffers are written on self.stream, so they come from its pool.  Taken from the pool of the staging
+    # thread's current stream (the compute stream) they could be blocks the embedder has freed while its kernels
+    # that use them are still queued there, and the decode of the next batch would race with them.
     def u8(self, s):
         if self.host_u8[s] is None:
             self.host_u8[s] = torch.empty(self.batch, self.H, self.W, 3, dtype=torch.uint8).pin_memory()
-            self.dev_u8[s] = torch.empty(self.batch, self.H, self.W, 3, dtype=torch.uint8, device=self.device)
+            with torch.cuda.stream(self.stream):
+                self.dev_u8[s] = torch.empty(self.batch, self.H, self.W, 3, dtype=torch.uint8, device=self.device)
         return self.host_u8[s], self.dev_u8[s]
 
     def f32(self, s):
         if self.dev_f32[s] is None:
-            self.dev_f32[s] = torch.empty(self.batch, 3, self.H, self.W, dtype=torch.float32, device=self.device,
-                                          memory_format=self.memory_format)
+            with torch.cuda.stream(self.stream):
+                self.dev_f32[s] = torch.empty(self.batch, 3, self.H, self.W, dtype=torch.float32, device=self.device,
+                                              memory_format=self.memory_format)
         return self.dev_f32[s]
 
     def check_status(self, s):
@@ -181,7 +186,9 @@ def _staging(batch, H, W, dev, fmt) -> "_Staging":
     st = _STAGING.get(key)
     if st is None:
         if len(_STAGING) >= 2:                               # e.g. the two magnifications of tree mode; no unbounded growth
-            _STAGING.pop(next(iter(_STAGING)))
+            old = _STAGING.pop(next(iter(_STAGING)))
+            for e in old.consumed:                           # its buffers return to its stream's pool: the compute
+                e.synchronize()                              # stream must have finished reading them
         st = _STAGING[key] = _Staging(batch, H, W, dev, fmt)
     st.status_names = [None, None]
     return st

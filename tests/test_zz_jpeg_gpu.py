@@ -200,3 +200,26 @@ def test_embed_bag_graph_replay_equals_eager_launches(tmp_path, monkeypatch):
     monkeypatch.setenv("DSMIL_B200_EMBED_GRAPH", "0")
     _, c_new_e = embed.embed_bag(paths, ic, batch_size=16, num_workers=2)
     assert torch.allclose(c_new, c_new_e, rtol=0, atol=1e-5) and not torch.allclose(c_new, c_g)
+
+
+def test_staging_buffers_come_from_the_staging_stream(tmp_path, monkeypatch):
+    """The staging thread writes the slot buffers on its own stream while the embedder runs on the compute stream.
+    Taken from the compute stream's pool, a slot could get a block the embedder has freed while its queued kernels
+    still use it, and the next batch's decode would race with them (rows of the second batch came out wrong)."""
+    import dsmil as mil
+    from dsmil_wsi_b200 import embed
+
+    class Tiny(torch.nn.Module):
+        def forward(self, x):
+            return x.mean(dim=(2, 3)).repeat(1, 4)
+    ic = mil.IClassifier(Tiny(), 12, 2).to(DEV).eval()
+    paths = embed.list_patches(_write_bag(tmp_path, 10, h=64, w=48))       # 3 batches of 4: both slots
+    for route in ("gpu", "host"):
+        monkeypatch.setenv("DSMIL_B200_JPEG", route)
+        embed.embed_bag(paths, ic, batch_size=4, num_workers=2)
+    st = next(s for s in embed._STAGING.values() if (s.batch, s.H, s.W) == (4, 64, 48))
+    torch.cuda.synchronize()
+    segments = torch.cuda.memory_snapshot()
+    for t in st.dev_f32 + st.dev_u8:
+        seg = next(g for g in segments if g["address"] <= t.data_ptr() < g["address"] + g["total_size"])
+        assert seg["stream"] == st.stream.cuda_stream
